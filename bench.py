@@ -45,6 +45,7 @@ DOC_TABLE = 65536                               # distinct synthetic documents' 
 CHUNK = 250_000                                 # corpus generation granularity (seed per global chunk)
 CE_CHUNK = int(os.environ.get("BENCH_CE_CHUNK", 800))      # rerank pairs per encoder call (117.6k tokens, ~2 GB of activations)
 PARITY_ROWS = 1_000_000                         # corpus block the in-run CPU-oracle parity check searches
+DUMP_BYTES = 64 << 20                           # cap on what --dump-outputs writes
 
 # BASELINE.json `configs` (SURVEY.md §8a: C2..C5) + the headline the metric is quoted on.  Every config runs on any
 # number of GPUs: the corpus is row-sharded over the ranks (strong scaling), rerank pairs are split over the ranks.
@@ -170,6 +171,19 @@ def models(W):
     ew = synthetic_bert_weights(ecfg, seed=0)
     cw = synthetic_bert_weights(ccfg, seed=1, with_head=True, scale=4.0)
     return ecfg, ccfg, ew, cw, PRESETS[W.emb][1]
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write the row-aligned [Q, k] result arrays as out_dir/<name>.npy.  Above DUMP_BYTES a fixed seeded sample
+    of rows is written, the same rows for the same arguments, so that two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a[0].nbytes for a in arrays.values())
+    rows = np.arange(n)
+    if n * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // row_bytes, replace=False))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[rows])
 
 
 def assemble_pairs_np(q_tok: np.ndarray, doc_tab: np.ndarray, ids: np.ndarray):
@@ -328,6 +342,8 @@ def run_gpu(args):
         out_ids, out_scores = step_device()
     ev1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"ids": out_ids.cpu().numpy().astype(np.float64), "scores": out_scores.cpu().numpy()})
     ms = torch.tensor([ev0.elapsed_time(ev1)], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -661,7 +677,14 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="headline", choices=sorted(CONFIGS),
                     help="BASELINE.json workload: headline (10M x 384, top-100, rerank), c2, c3, c4, c5")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write the last step's result to DIR: ids.npy (float64 corpus row ids, "
+                         "best first) and scores.npy (float32 rerank logits, or top-k scores without rerank), both [Q, k]")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

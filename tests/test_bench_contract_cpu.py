@@ -23,3 +23,21 @@ def test_reference_arm_prints_the_contract_line():
     cb = d["cpu_baseline"]
     assert cb["kind"] in ("port", "reference") and cb["cores"] >= 1 and cb["value"] == d["value"] and cb["sample"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_dump_outputs_caps_the_size_with_a_fixed_row_sample(tmp_path, monkeypatch):
+    import numpy as np
+
+    import bench
+    ids = np.arange(4000, dtype=np.float64).reshape(400, 10)
+    sc = -ids.astype(np.float32)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100 * 10 * (8 + 4))
+    for sub in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / sub), {"ids": ids, "scores": sc})
+    a_ids, a_sc = np.load(tmp_path / "a" / "ids.npy"), np.load(tmp_path / "a" / "scores.npy")
+    assert a_ids.shape == a_sc.shape == (100, 10) and a_ids.nbytes + a_sc.nbytes <= bench.DUMP_BYTES
+    rows = (a_ids[:, 0] // 10).astype(int)
+    assert (np.diff(rows) > 0).all() and (a_ids == ids[rows]).all() and (a_sc == sc[rows]).all()
+    assert np.array_equal(a_ids, np.load(tmp_path / "b" / "ids.npy"))
+    bench.dump_outputs(str(tmp_path / "small"), {"ids": ids[:5], "scores": sc[:5]})      # under the cap: every row
+    assert np.array_equal(np.load(tmp_path / "small" / "ids.npy"), ids[:5])
