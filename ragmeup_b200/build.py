@@ -18,9 +18,11 @@ SOURCES = ["rmu_common.cu", "rmu_index.cu", "rmu_gemm.cu", "rmu_encoder.cu", "rm
 # every header under csrc/ takes part in the up-to-date check (a list kept by hand once missed rmu_attention.cuh / rmu_scan.cuh)
 HEADERS = sorted(f for f in os.listdir(CSRC) if f.endswith((".cuh", ".h"))) + [os.path.join("..", "..", "include", "ragmeup_b200.h")]
 
+# -compress-all: by default the fatbinary is compressed only past a size threshold, so which object files came out
+# compressed depended on how many kernel instantiations they held
 NVCC_FLAGS = [
     "-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
-    "-Xcompiler", "-fPIC", "-Xcompiler", "-O3", "--diag-suppress", "550",
+    "-Xcompiler", "-fPIC", "-Xcompiler", "-O3", "--diag-suppress", "550", "-Xfatbin", "-compress-all",
 ]
 
 

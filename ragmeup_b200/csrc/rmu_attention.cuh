@@ -397,17 +397,7 @@ struct ApParams {
     int B, heads, H;
     int kp;                 // rows per K / V plane of a slot: max_seqlen rounded up to 32 (<= kApMaxKeys)
     __half* ctx_hi; __half* ctx_lo;
-    unsigned long long* trace;      // study (RMU_ATTN_TRACE=1): per-role event lanes of CTA 0, (event << 48 | arg << 32 | clock)
 };
-
-// study: one store per event into the calling role's own lane of the buffer (no atomics: an atomic's round trip would
-// stall the single-thread issuers the trace is meant to observe)
-constexpr int kApTraceRoles = 12, kApTraceLen = 1024;
-__device__ __forceinline__ void ap_trace(const ApParams& p, int role, uint32_t& tn, unsigned ev, unsigned arg) {
-    if (p.trace != nullptr && blockIdx.x == 0 && tn < static_cast<uint32_t>(kApTraceLen))
-        p.trace[role * kApTraceLen + tn++] = (static_cast<unsigned long long>(ev) << 48) | (static_cast<unsigned long long>(arg & 0xFFFF) << 32) |
-                                             (static_cast<unsigned long long>(clock64()) & 0xFFFFFFFFull);
-}
 
 // packed fp32 pairs (FADD2 / FFMA2 of sm_100): one issue slot for two lanes' worth of softmax arithmetic
 __device__ __forceinline__ void ap_add2(float& x0, float& x1, float y0, float y1) {
@@ -471,7 +461,6 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap t_qkv, const ApParams 
     const unsigned lane = lane_id();
     const int hpairs = p.heads >> 1;
     const int nwork = p.B * hpairs;
-    uint32_t tn = 0;                                       // trace entries this thread has written
 
     if (threadIdx.x == 0) {
         for (int i = 0; i < 2; ++i) {
@@ -502,7 +491,6 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap t_qkv, const ApParams 
                 mbar_wait(&kv_empty[kvs], ((kvi >> 1) & 1) ^ 1);
                 const int nkb = (S + 31) >> 5;
                 uint8_t* kb0 = kvring + kvs * kvslot;
-                ap_trace(p, 0, tn, 1, kvi);
                 mbar_arrive_expect_tx(&kv_full[kvs], static_cast<uint32_t>(4 * nkb * 32 * kApRowB));
                 for (int kb = 0; kb < nkb; ++kb) {
                     uint8_t* d = kb0 + kb * 32 * kApRowB;
@@ -516,7 +504,6 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap t_qkv, const ApParams 
                     mbar_wait(&q_empty[qs], ((qi >> 1) & 1) ^ 1);
                     const int nqb = (min(kAtcRows, S - r0) + 31) >> 5;
                     uint8_t* q0 = qring + qs * kApQSlot;
-                    ap_trace(p, 0, tn, 2, qi);
                     mbar_arrive_expect_tx(&q_full[qs], static_cast<uint32_t>(2 * nqb * 32 * kApRowB));
                     for (int qb = 0; qb < nqb; ++qb) {
                         tma_load_2d(q0 + qb * 32 * kApRowB, &t_qkv, col, t0 + r0 + qb * 32, &q_full[qs], kEvictNormal);
@@ -541,13 +528,11 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap t_qkv, const ApParams 
                 for (int r0 = 0; r0 < S; r0 += kAtcRows, ++qi, ++cnt) {
                     const int qs = qi & 1;
                     mbar_wait(&q_full[qs], (qi >> 1) & 1);
-                    ap_trace(p, 1, tn, 3, cnt);
                     const uint32_t qbase = smem_u32(qring + qs * kApQSlot);
 #pragma unroll
                     for (int g = 0; g < 2; ++g) {
                         mbar_wait(&s_free[g], (cnt & 1) ^ 1);    // P V of this head's previous tile no longer reads the buffer
                         tc_fence_after();
-                        ap_trace(p, 1, tn, 4 + g, cnt);
                         const uint32_t d_addr = tmem_base + g * kAtcBufCols;
                         const uint32_t qg = qbase + g * kAtcRows * kApRowB, kg = kbase + g * kvplane;   // rows = [hi 64 B | lo 64 B]
 #pragma unroll
@@ -559,7 +544,6 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap t_qkv, const ApParams 
                                            (term | k) != 0 ? 1u : 0u);
                         }
                         tc_commit(&s_full[g]);
-                        ap_trace(p, 1, tn, 6 + g, cnt);
                     }
                     tc_commit(&q_empty[qs]);                     // the Q tile has been read by both heads' MMAs
                 }
@@ -587,7 +571,6 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap t_qkv, const ApParams 
                         ppar ^= 1u << c;
                         if (c == 0) mbar_wait(&o_free[g], (cnt & 1) ^ 1);   // the output warps have read the previous tile's O
                         tc_fence_after();
-                        ap_trace(p, 2 + g, tn, 10 + g, c);
                         for (int j16 = 2 * c; j16 < min(2 * c + 2, nk16); ++j16) {
                             const uint32_t a_hi = pbase + 32 * c + 8 * (j16 & 1), a_lo = a_hi + 16;
                             const uint64_t bv = atc_desc(vg + j16 * 16 * kApRowB, SBO, LAYOUT);
@@ -595,7 +578,6 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap t_qkv, const ApParams 
                             mma_f16_ts(d0, a_hi, bv, IDESC_O64, acc);
                             mma_f16_ts(d0, a_lo, bv, IDESC_O32, 1u);      // N = 32: lands on the V_hi half of the same accumulator
                         }
-                        ap_trace(p, 2 + g, tn, 12 + g, c);
                     }
                     tc_commit(&o_full[g]);
                     tc_commit(&s_free[g]);
@@ -622,7 +604,6 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap t_qkv, const ApParams 
                     const float inv = 1.0f / (lp[r] + lp[kAtcRows + r]);
                     mbar_wait(&o_full[g], cnt & 1);
                     tc_fence_after();
-                    if (lane == 0) ap_trace(p, 8 + quad, tn, 26 + g, cnt);
                     const uint32_t ob = tmem_addr(tmem_base, quad * 32, g * kAtcBufCols + OCOL);
                     uint32_t oh[16], ol[16];
                     if (warp_live) {
@@ -653,7 +634,6 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap t_qkv, const ApParams 
                             dl[q] = make_uint4(ol[4 * q], ol[4 * q + 1], ol[4 * q + 2], ol[4 * q + 3]);
                         }
                     }
-                    if (lane == 0) ap_trace(p, 8 + quad, tn, 28 + g, cnt);
                 }
             }
         }
@@ -676,7 +656,6 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap t_qkv, const ApParams 
                 const bool warp_live = r0 + quad * 32 < S;
                 mbar_wait(&s_full[g], cnt & 1);
                 tc_fence_after();
-                if (htid == 0) ap_trace(p, 4 + g + 2 * half, tn, 20 + g, cnt);
                 float m = -INFINITY;
                 if (warp_live) {
                     float m1 = -INFINITY, m2 = -INFINITY, m3 = -INFINITY;   // four independent chains: fmaxf does not reassociate
@@ -701,7 +680,6 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap t_qkv, const ApParams 
                 bar_sync_named(1 + g * 4 + quad, 64);            // the two warps that share these 32 rows (same SM sub-partition)
                 m = fmaxf(m, xo[r]);
                 bar_sync_named(1 + g * 4 + quad, 64);
-                if (htid == 0) ap_trace(p, 4 + g + 2 * half, tn, 22 + g, cnt);
                 float l0 = 0.f, l1 = 0.f;
                 for (int c = half; c < nchunk; c += 2) {
                     if (warp_live) {
@@ -731,7 +709,6 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap t_qkv, const ApParams 
                     tc_fence_before();
                     __syncwarp();
                     if (lane == 0) mbar_arrive(&p_full[g * kAtcMaxChunks + c]);     // one arrival per owning warp: no CTA-level barrier
-                    if (htid == 0) ap_trace(p, 4 + g + 2 * half, tn, 24 + g, c);
                 }
                 xm[r] = l0 + l1;                                 // row sum for the output warps (every warp of the head is past pass 1)
                 mbar_arrive(&l_full[g]);

@@ -13,7 +13,6 @@
 // Activations between kernels are split fp16 planes (see rmu_gemm.cuh); LayerNorm, softmax, GELU,
 // residual adds, pooling and the classifier head are fp32.
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 #include <vector>
 
@@ -152,7 +151,7 @@ constexpr int kKeySB = 256;   // keys resident in shared memory at a time
 // attention_planes_kernel (mma.sync; sequences the tcgen05 kernel does not take): Q (pre-scaled), K and V arrive as
 // split fp16 planes [T, 3H] written by the QKV GEMM epilogue, so this kernel does no conversion work:
 // K / V tiles are 16-byte copies into shared memory ([key][d] for both) and the P V operand is fetched
-// with ldmatrix.trans.  One CTA = (sequence, head, block of 16*NW query rows), one warp = 16 rows.
+// with ldmatrix.trans.  One CTA = (sequence, head, block of 16 * kAttWarps query rows), one warp = 16 rows.
 // ---------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void ldmatrix_x4_trans(uint32_t (&r)[4], const void* smem_row) {
     asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
@@ -178,8 +177,8 @@ __device__ __forceinline__ float fast_exp2(float x) {   // ex2.approx: 2 ulp, ex
 // to 3 CTAs / 64 registers spills in the key loop and measured 541 us instead of 352 us per layer call).
 // Grid = (heads, sequences, row blocks): the heads of one sequence run together, so the 64-byte (d_h = 32)
 // K / V row segments of neighbouring heads are fetched from DRAM as whole lines.
-template <int DH, int MINB, int NW = kAttWarps>      // NW warps = 16 * NW query rows per CTA
-__global__ void __launch_bounds__(NW * 32, MINB) attention_planes_kernel(const __half* __restrict__ ph, const __half* __restrict__ pl,
+template <int DH, int MINB>
+__global__ void __launch_bounds__(kAttWarps * 32, MINB) attention_planes_kernel(const __half* __restrict__ ph, const __half* __restrict__ pl,
                                                                           const int* __restrict__ cu, int H, int ksb,
                                                                           __half* __restrict__ ctx_hi, __half* __restrict__ ctx_lo) {
     constexpr int KSTR = DH + 8;
@@ -193,7 +192,7 @@ __global__ void __launch_bounds__(NW * 32, MINB) attention_planes_kernel(const _
 
     const int b = blockIdx.y, h = blockIdx.x;
     const int t0 = cu[b], S = cu[b + 1] - t0;
-    const int rbase = blockIdx.z * (NW * 16);
+    const int rbase = blockIdx.z * (kAttWarps * 16);
     if (rbase >= S) return;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
     const size_t ld = static_cast<size_t>(3) * H;
@@ -582,23 +581,20 @@ static int run_encoder(rmu_encoder* e, const int32_t* ids, const int32_t* type_i
     const float scale = 1.0f / sqrtf(static_cast<float>(DH));
     for (int l = 0; l < c.layers; ++l) {
         EncLayer& L = e->layers[l];
-        // RMU_ATTN_MODE: 0 = tcgen05 attention where the shape allows it (head-pair kernel, else per-head kernel, else mma.sync),
-        // 1 = never the head-pair kernel, 3 = always mma.sync
-        static const int attn_mode = [] { const char* e = getenv("RMU_ATTN_MODE"); return e ? atoi(e) : 0; }();
         GemmParams g{};
         g.M = T; g.N = 3 * H; g.K = H; g.bias = L.bqkv;
         // q (scaled by 1/sqrt(dh)), k, v leave the GEMM as split fp16 planes: attention does no conversions
         // (the softmax runs in base 2: q also carries log2(e))
         g.out_hi = e->QKVP.hi; g.out_lo = e->QKVP.lo; g.qcols = H; g.qscale = scale * 1.4426950408889634f;
         // the head-pair attention kernel reads q / k / v with hi and lo of a head interleaved in one 128-byte line
-        const bool pair_attn = attn_mode == 0 && DH == 32 && c.heads % 2 == 0 && max_seqlen <= kApMaxKeys;
+        const bool pair_attn = DH == 32 && c.heads % 2 == 0 && max_seqlen <= kApMaxKeys;
         if (pair_attn) { g.out_hi = e->QKVI; g.out_lo = nullptr; g.interleave32 = 1; }
         rc = launch_gemm(GEMM_BIAS_SPLIT_QSCALE, e->X, L.Wqkv, g, e->sms, st);
         if (rc != RMU_OK) return rc;
         {
             ProfScope _ps(PROF_ATTN, st);
             // tcgen05 attention: all keys of a sequence in one TMEM score tile (<= 256 - d_h keys) and at least two operand
-            // slots in shared memory; longer sequences take the mma.sync kernel (RMU_ATTN_MODE=3 forces it)
+            // slots in shared memory; longer sequences take the mma.sync kernel
             const int kp = (max_seqlen + 63) / 64 * 64;
             const int slot_bytes = 2 * kAtcRows * DH * 2 + 4 * kp * DH * 2;
             const int nslots = std::min(kAtcMaxSlots, (227 * 1024 - 1024 - kAtcStateBytes) / slot_bytes);
@@ -612,27 +608,8 @@ static int run_encoder(rmu_encoder* e, const int32_t* ids, const int32_t* type_i
                 const long long nwork = static_cast<long long>(B) * (c.heads / 2);
                 const unsigned grid = static_cast<unsigned>(std::min<long long>(e->sms, nwork));
                 RMU_CUDA(cudaFuncSetAttribute(attention_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-                static const int att_trace = [] { const char* e = getenv("RMU_ATTN_TRACE"); return e ? atoi(e) : 0; }();
-                static unsigned long long* trace_buf = nullptr;
-                constexpr size_t trace_n = static_cast<size_t>(kApTraceRoles) * kApTraceLen;
-                if (att_trace && l == 1) {                           // study: event timeline of CTA 0, second layer of a call
-                    if (!trace_buf) cudaMalloc(reinterpret_cast<void**>(&trace_buf), trace_n * sizeof(unsigned long long));
-                    cudaMemsetAsync(trace_buf, 0, trace_n * sizeof(unsigned long long), st);
-                    ap.trace = trace_buf;
-                }
                 attention_pair_kernel<<<grid, kApThreads, smem, st>>>(e->att_qkvi, ap);
-                if (att_trace && l == 1) {
-                    std::vector<unsigned long long> h(trace_n);
-                    cudaMemcpyAsync(h.data(), trace_buf, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st);
-                    cudaStreamSynchronize(st);
-                    FILE* f = fopen("gpurun_out/att_trace.txt", "w");
-                    if (f) {
-                        for (size_t i = 0; i < trace_n; ++i)
-                            if (h[i] != 0) fprintf(f, "%llu %llu %llu\n", h[i] >> 48, (h[i] >> 32) & 0xFFFF, h[i] & 0xFFFFFFFFull);
-                        fclose(f);
-                    }
-                }
-            } else if ((attn_mode == 0 || attn_mode == 1) && max_seqlen <= kAtcBufCols - DH && nslots >= 2) {
+            } else if (max_seqlen <= kAtcBufCols - DH && nslots >= 2) {
                 AtcParams ap{};
                 ap.cu = cu; ap.B = B; ap.heads = c.heads; ap.H = H; ap.row_tiles = (max_seqlen + kAtcRows - 1) / kAtcRows;
                 ap.kp = kp; ap.nslots = nslots; ap.ctx_hi = e->CTX.hi; ap.ctx_lo = e->CTX.lo;
@@ -649,19 +626,15 @@ static int run_encoder(rmu_encoder* e, const int32_t* ids, const int32_t* type_i
                     attention_tc_kernel<64><<<grid, kAtcThreads, smem, st>>>(e->att_q_hi, e->att_q_lo, e->att_k_hi, e->att_k_lo, ap);
                 }
             } else {
-                // RMU_ATTN_WARPS = 5: 80-row CTAs, four per SM (same warps/SM, K/V staged twice per 147-token sequence)
-                static const int nw_env = [] { const char* e = getenv("RMU_ATTN_WARPS"); return e ? atoi(e) : kAttWarps; }();
-                const int nw = (nw_env == 5 && DH == 32) ? 5 : kAttWarps;
                 dim3 pg(static_cast<unsigned>(c.heads), static_cast<unsigned>(B),
-                        static_cast<unsigned>((max_seqlen + nw * 16 - 1) / (nw * 16)));
+                        static_cast<unsigned>((max_seqlen + kAttWarps * 16 - 1) / (kAttWarps * 16)));
                 // keys resident per CTA: the whole (longest) sequence when it fits, else super-blocks of kKeySB
                 const int ksb = std::min(kKeySB, (max_seqlen + 31) / 32 * 32);
                 const size_t smem_max = 4 * sizeof(__half) * static_cast<size_t>(kKeySB) * (DH + 8);
                 const size_t smem = 4 * sizeof(__half) * static_cast<size_t>(ksb) * (DH + 8);
-                auto kern = DH == 32 ? (nw == 5 ? attention_planes_kernel<32, 4, 5> : attention_planes_kernel<32, 2>)
-                                     : attention_planes_kernel<64, 1>;   // d_h = 64 needs > 96 registers
+                auto kern = DH == 32 ? attention_planes_kernel<32, 2> : attention_planes_kernel<64, 1>;   // d_h = 64 needs > 96 registers
                 RMU_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem_max)));
-                kern<<<pg, nw * 32, smem, st>>>(e->QKVP.hi, e->QKVP.lo, cu, H, ksb, e->CTX.hi, e->CTX.lo);
+                kern<<<pg, kAttWarps * 32, smem, st>>>(e->QKVP.hi, e->QKVP.lo, cu, H, ksb, e->CTX.hi, e->CTX.lo);
             }
         }
         count_launch();

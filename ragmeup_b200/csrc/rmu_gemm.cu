@@ -1,5 +1,4 @@
 #include <algorithm>
-#include <cstdlib>
 
 #include "rmu_gemm.cuh"
 
@@ -37,13 +36,11 @@ static int launch_bn(const SplitOperand& A, const SplitOperand& W, const GemmPar
     return RMU_OK;
 }
 
-// tile width: RMU_GEMM_BN = 128 | 192 | 256 forces one (when it divides N); default 192, else 256, else 128
+// tile width: 192 when it divides N, else 256, else 128
 template <int MODE>
 static int launch_mode(const SplitOperand& A, const SplitOperand& W, const GemmParams& p, int sms, cudaStream_t st) {
-    static const int force = [] { const char* e = getenv("RMU_GEMM_BN"); return e ? atoi(e) : 0; }();
     int bn = 128;
-    if (force == 128 || force == 192 || force == 256) { if (p.N % force == 0) bn = force; }
-    else if (p.N % 192 == 0) bn = 192;      // measured best on the MiniLM / bge shapes (768, 1152, 1536, 2304, 3072 ...)
+    if (p.N % 192 == 0) bn = 192;           // measured best on the MiniLM / bge shapes (768, 1152, 1536, 2304, 3072 ...)
     else if (p.N % 256 == 0) bn = 256;
     if (!W.is_weight) bn = 128;              // operand without the wide weight maps
     if (bn == 256) return launch_bn<MODE, 256>(A, W, p, sms, st);
@@ -52,8 +49,7 @@ static int launch_mode(const SplitOperand& A, const SplitOperand& W, const GemmP
 }
 
 bool gemm_ln_supported(const SplitOperand& W, int N) {
-    static const int off = [] { const char* e = getenv("RMU_LN_FUSED"); return e ? atoi(e) == 0 : 0; }();
-    return !off && W.is_weight && (N == 2 * kLnBN || N == 4 * kLnBN);
+    return W.is_weight && (N == 2 * kLnBN || N == 4 * kLnBN);
 }
 
 int launch_gemm_ln(const SplitOperand& A, const SplitOperand& W, const GemmLnParams& p_in, int sms, cudaStream_t st) {
@@ -65,9 +61,8 @@ int launch_gemm_ln(const SplitOperand& A, const SplitOperand& W, const GemmLnPar
     }
     const int CL = p.N / kLnBN;
     // three epilogue warps per TMEM lane quadrant when the projection is short (K <= 512: its epilogue, not its MMAs,
-    // bounds it: 158 -> 145 us at K = 384) and the cluster is a pair (shared-memory budget); RMU_LN_EPI = 8 | 12 forces
-    static const int epi_env = [] { const char* e = getenv("RMU_LN_EPI"); return e ? atoi(e) : 0; }();
-    const bool epi12 = CL == 2 && (epi_env == 12 || (epi_env == 0 && p.K <= 512));
+    // bounds it: 158 -> 145 us at K = 384) and the cluster is a pair (shared-memory budget)
+    const bool epi12 = CL == 2 && p.K <= 512;
     if (epi12) RMU_CUDA(cudaFuncSetAttribute(gemm_f16x3_ln_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ln_smem_bytes(12))));
     else RMU_CUDA(cudaFuncSetAttribute(gemm_f16x3_ln_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ln_smem_bytes(8))));
     const int m_blks = (p.M + kGemmBM - 1) / kGemmBM;
@@ -92,17 +87,13 @@ int launch_gemm_ln(const SplitOperand& A, const SplitOperand& W, const GemmLnPar
     return RMU_OK;
 }
 
-int launch_gemm(int mode, const SplitOperand& A, const SplitOperand& W, const GemmParams& p_in, int sms, cudaStream_t st) {
-    static const int ablate = [] { const char* e = getenv("RMU_GEMM_ABLATE"); return e ? atoi(e) : 0; }();
-    GemmParams p = p_in;
-    p.ablate = ablate;
+int launch_gemm(int mode, const SplitOperand& A, const SplitOperand& W, const GemmParams& p, int sms, cudaStream_t st) {
     if (p.M <= 0) return RMU_OK;
     if (p.N % 128 != 0 || p.K % kGemmBK != 0 || A.cols != p.K || W.cols != p.K || W.rows < p.N || A.rows < p.M) {
         set_error("launch_gemm: shape not supported (N % 128, K % 64)");
         return RMU_ERR_UNSUPPORTED;
     }
     switch (mode) {
-        case GEMM_BIAS_F32: return launch_mode<GEMM_BIAS_F32>(A, W, p, sms, st);
         case GEMM_BIAS_GELU_SPLIT: return launch_mode<GEMM_BIAS_GELU_SPLIT>(A, W, p, sms, st);
         case GEMM_BIAS_RESID_F32: return launch_mode<GEMM_BIAS_RESID_F32>(A, W, p, sms, st);
         case GEMM_BIAS_SPLIT_QSCALE: return launch_mode<GEMM_BIAS_SPLIT_QSCALE>(A, W, p, sms, st);

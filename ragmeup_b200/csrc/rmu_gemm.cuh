@@ -27,7 +27,6 @@ constexpr size_t kGemmStagingBytes = static_cast<size_t>(kGemmEpiWarps) * 32 * k
 constexpr size_t kGemmSmem = 196608 + kGemmStagingBytes + 256 + 1024;   // stages never exceed 192 KB
 
 enum GemmMode {
-    GEMM_BIAS_F32 = 0,        // out_f32 = acc + bias
     GEMM_BIAS_GELU_SPLIT = 1, // out planes = split(gelu_erf(acc + bias))
     GEMM_BIAS_RESID_F32 = 2,  // out_f32 = acc + bias + (res_hi + res_lo)
     GEMM_BIAS_SPLIT_QSCALE = 3, // out planes = split((acc + bias) * (col < qcols ? qscale : 1))   (QKV projection)
@@ -43,8 +42,6 @@ struct GemmParams {
     int interleave32;                     // GEMM_BIAS_SPLIT_QSCALE: out_hi is ONE buffer [M, 2N] where every 32-column group
                                           // (a d_h = 32 head) is stored as 32 hi halves followed by its 32 lo halves: a head's
                                           // q / k / v row is one 128-byte line (what attention_pair_kernel's TMA boxes fetch)
-    int ablate;                           // RMU_GEMM_ABLATE (profiling only, results are wrong): 1 skip the MMAs, 2 skip the TMA
-                                          // loads, 4 skip the epilogue's arithmetic and stores
 };
 
 __device__ __forceinline__ void split_f16(float v, __half& hi, __half& lo) {
@@ -187,7 +184,6 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap tAh, const __grid_constant
                 for (int kb = 0; kb < k_blks; ++kb) {
                     mbar_wait(&empty[slot], phase ^ 1);
                     uint8_t* st = smem + slot * kGemmStageBytes;
-                    if (p.ablate & 2) { mbar_arrive(&full[slot]); if (++slot == kGemmStages) { slot = 0; phase ^= 1; } continue; }
                     mbar_arrive_expect_tx(&full[slot], kGemmStageBytes);
                     tma_load_2d(st, &tAh, kb * kGemmBK, mb * kGemmBM, &full[slot], kEvictNormal);
                     tma_load_2d(st + kGemmPlaneBytes, &tAl, kb * kGemmBK, mb * kGemmBM, &full[slot], kEvictNormal);
@@ -218,7 +214,6 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap tAh, const __grid_constant
                     const uint64_t dWl = umma_desc_sw128_kmajor(sbase + 2 * kGemmPlaneBytes + kWPlane);
 #pragma unroll
                     for (int k = 0; k < kGemmBK / 16; ++k) {
-                        if (p.ablate & 1) break;
                         const uint64_t off = static_cast<uint64_t>(k * 2);   // 16 halves = 32 B = 2 x 16 B units
                         mma_f16_ss(d_addr, dAh + off, dWh + off, IDESC, (kb | k) != 0 ? 1u : 0u);
                         mma_f16_ss(d_addr, dAl + off, dWh + off, IDESC, 1u);
@@ -273,7 +268,6 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap tAh, const __grid_constant
                     mbar_arrive(&acc_empty[buf]);
                 }
                 const float sc = (MODE == GEMM_BIAS_SPLIT_QSCALE && col0 < p.qcols) ? p.qscale : 1.0f;
-                if (p.ablate & 4) continue;
 #pragma unroll
                 for (int j = 0; j < 32; ++j) stg[lane * kGemmStageRow + j] = __uint_as_float(r[j]);
                 __syncwarp();
@@ -289,7 +283,7 @@ gemm_f16x3_kernel(const __grid_constant__ CUtensorMap tAh, const __grid_constant
                         const size_t o = static_cast<size_t>(grow) * p.N + col0 + cp;
                         if (MODE == GEMM_BIAS_RESID_F32)
                             v = f2_add(v, f2_add(__half22float2(rsh[rr >> 1]), __half22float2(rsl[rr >> 1])));
-                        if (MODE == GEMM_BIAS_F32 || MODE == GEMM_BIAS_RESID_F32) {
+                        if (MODE == GEMM_BIAS_RESID_F32) {
                             *reinterpret_cast<float2*>(p.out_f32 + o) = v;
                         } else {
                             __half2 h2, l2;

@@ -16,7 +16,6 @@
 //              does not take) run the exact fp32 CUDA-core scan.
 // The ids and scores returned are therefore those of an exact fp32 brute-force search.
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 #include <vector>
 
@@ -672,16 +671,9 @@ struct ScanGeom { int nq, nstages, pair; size_t smem; };
 constexpr int kPass2MaxQ = 256;         // flagged queries the second pass takes per search (more stay flagged)
 constexpr int kPass2PoolCap = 16384;    // rows a flagged query may collect; more -> the exact scan answers
 
-static int env_int(const char* name, int dflt) { const char* e = getenv(name); return e ? atoi(e) : dflt; }
-static int scan_kd() { static const int v = env_int("RMU_SCAN_KD", 2) == 1 ? 1 : 2; return v; }          // boxes per stage
-// RMU_SCAN_PAIR: 1 = always the cta_group::2 kernel, 0 = never, unset = when it saves a pass over the corpus
-static int scan_pair_mode() { static const int v = env_int("RMU_SCAN_PAIR", -1); return v; }
-static int scan_stages_cap() { static const int v = env_int("RMU_SCAN_STAGES", 0); return v; }           // study: cap the ring
-static int scan_ablate() { static const int v = env_int("RMU_SCAN_ABLATE", 0); return v; }
-
-template <int NQ, int KD, bool PAIR>
+template <int NQ, bool PAIR>
 static int scan_launch_t(const CUtensorMap& tx, const CUtensorMap& tq, const ScanParams& p, int grid, size_t smem, cudaStream_t st) {
-    auto kern = scan_rows_kernel<NQ, KD, PAIR>;
+    auto kern = scan_rows_kernel<NQ, PAIR>;
     // per device and cheap: set on every launch (a process may drive several GPUs); always the device maximum, so that
     // concurrent callers on other handles never lower it under a launch that needs more
     RMU_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
@@ -702,14 +694,10 @@ static int scan_launch_t(const CUtensorMap& tx, const CUtensorMap& tq, const Sca
 }
 
 static int scan_dispatch(const ScanGeom& g, const CUtensorMap& tx, const CUtensorMap& tq, const ScanParams& p, int grid, cudaStream_t st) {
-    const int kd = scan_kd();
-#define RMU_SCAN_CASE(NQ)                                                                                        \
-    if (g.nq == NQ) {                                                                                            \
-        if (g.pair) return kd == 2 ? scan_launch_t<NQ, 2, true>(tx, tq, p, grid, g.smem, st) : scan_launch_t<NQ, 1, true>(tx, tq, p, grid, g.smem, st);   \
-        return kd == 2 ? scan_launch_t<NQ, 2, false>(tx, tq, p, grid, g.smem, st) : scan_launch_t<NQ, 1, false>(tx, tq, p, grid, g.smem, st);             \
-    }
-    RMU_SCAN_CASE(128) RMU_SCAN_CASE(64) RMU_SCAN_CASE(32) RMU_SCAN_CASE(16)
-#undef RMU_SCAN_CASE
+#define SCAN_CASE(NQ)                                                                                            \
+    if (g.nq == NQ) return g.pair ? scan_launch_t<NQ, true>(tx, tq, p, grid, g.smem, st) : scan_launch_t<NQ, false>(tx, tq, p, grid, g.smem, st);
+    SCAN_CASE(128) SCAN_CASE(64) SCAN_CASE(32) SCAN_CASE(16)
+#undef SCAN_CASE
     set_error("scan: unsupported geometry");
     return RMU_ERR_UNSUPPORTED;
 }
@@ -721,7 +709,7 @@ static int scan_block_cap(int dim, bool pair) {
     while (cap >= 16 && KB * (cap / (pair ? 2 : 1)) * 128 > kScanQOpMax) cap >>= 1;
     return cap >= 16 ? cap : 0;
 }
-static int scan_max_block(int dim) { return std::max(scan_block_cap(dim, false), scan_pair_mode() != 0 ? scan_block_cap(dim, true) : 0); }
+static int scan_max_block(int dim) { return std::max(scan_block_cap(dim, false), scan_block_cap(dim, true)); }
 
 // geometry for `rem` queries still to scan.  Single CTAs keep the whole query block resident (<= 64 queries at 384
 // dims) and are the faster kernel per pass (measured 10M x 384, Q = 64: 2.26 ms vs 2.36 ms); CTA pairs keep half a
@@ -731,18 +719,35 @@ static ScanGeom scan_geometry(int dim, int rem) {
     const int KB = (dim + 31) / 32;
     const int cap1 = scan_block_cap(dim, false), cap2 = scan_block_cap(dim, true);
     ScanGeom g{};
-    g.pair = scan_pair_mode() == 1 || cap1 == 0 || (scan_pair_mode() != 0 && rem > cap1 && cap2 > cap1);
+    g.pair = cap1 == 0 || (rem > cap1 && cap2 > cap1);
     const int cap = g.pair ? cap2 : cap1;
     int nq = 16;
     while (nq < cap && nq < rem) nq <<= 1;
     const size_t qop = static_cast<size_t>(KB) * (nq / (g.pair ? 2 : 1)) * 128;
-    const size_t stage = static_cast<size_t>(scan_kd()) * kBoxBytes;
+    const size_t stage = static_cast<size_t>(kScanKD) * kBoxBytes;
     const size_t budget = 227 * 1024 - 1024 - kScanStateBytes - qop;
     g.nq = nq;
     g.nstages = static_cast<int>(std::min<size_t>(budget / stage, kScanMaxStages));
-    if (scan_stages_cap() > 0) g.nstages = std::min(g.nstages, scan_stages_cap());
     g.smem = 1024 + qop + static_cast<size_t>(g.nstages) * stage + kScanStateBytes;
     return g;
+}
+
+// one scan launch over the first `ntiles` corpus tiles for the nq queries at qbase (row pitch = dim), one CTA per SM.
+// `sp` comes with the fields of the caller's pass set; the ones every launch shares are filled here.  Grids too small
+// for the threshold exchange run without it (sp.groups = 0).  *grid_out (if given) receives the grid.
+static int scan_launch(rmu_index* idx, const ScanGeom& geo, const float* qbase, int nq, int ntiles, ScanParams& sp,
+                       cudaStream_t st, int* grid_out = nullptr) {
+    const int D = idx->dim;
+    const int grid = geo.pair ? 2 * std::min(idx->sms / 2, (ntiles + 1) / 2) : std::min(idx->sms, ntiles);
+    CUtensorMap tq;
+    const int rc = make_tmap_2d(&tq, qbase, static_cast<uint64_t>(nq), static_cast<uint64_t>(D),
+                                static_cast<uint64_t>(D) * sizeof(float), 32, static_cast<uint32_t>(geo.nq / (geo.pair ? 2 : 1)), 4);
+    if (rc != RMU_OK) return rc;
+    sp.nq = nq; sp.dim = D; sp.n = idx->n; sp.ntiles = ntiles; sp.nstages = geo.nstages; sp.metric = idx->metric;
+    sp.rscale = idx->rscale; sp.rbias = idx->rbias; sp.stats_bits = idx->max_norm_bits; sp.gmax = idx->gmax;
+    if (grid < 2 * sp.groups) sp.groups = 0;         // small grids: lists are cut only by their own floors
+    if (grid_out) *grid_out = grid;
+    return scan_dispatch(geo, idx->tmap, tq, sp, grid, st);
 }
 
 extern "C" {
@@ -943,17 +948,9 @@ int rmu_index_search(rmu_index* idx, const float* queries, int nq, int k, int64_
         for (int q0 = 0; q0 < nq;) {
             const ScanGeom geo = scan_geometry(D, nq - q0);
             const int nql = std::min(nq - q0, geo.nq);
-            const int grid = geo.pair ? 2 * std::min(idx->sms / 2, (ntiles + 1) / 2) : std::min(idx->sms, ntiles);   // one CTA per SM
             const float* qbase = queries + static_cast<size_t>(q0) * D;
-            CUtensorMap tq;
-            rc = make_tmap_2d(&tq, qbase, static_cast<uint64_t>(nql), static_cast<uint64_t>(D),
-                              static_cast<uint64_t>(D) * sizeof(float), 32, static_cast<uint32_t>(geo.nq / (geo.pair ? 2 : 1)), 4);
-            if (rc != RMU_OK) return rc;
             ScanParams sp{};
-            sp.ablate = scan_ablate();
-            sp.nq = nql; sp.dim = D; sp.n = N; sp.ntiles = ntiles; sp.nstages = geo.nstages; sp.metric = idx->metric;
-            sp.rscale = idx->rscale; sp.rbias = idx->rbias; sp.stats_bits = idx->max_norm_bits;
-            sp.lists = d_scan; sp.counts = d_cnt; sp.floors = d_floor; sp.gmax = idx->gmax;
+            sp.lists = d_scan; sp.counts = d_cnt; sp.floors = d_floor;
             sp.epoch = ++idx->epoch;
             if (idx->epoch == 0xFFFFFFFFu) {                 // epoch wrap: start over from clean tags
                 RMU_CUDA(cudaMemsetAsync(idx->gmax, 0, sizeof(unsigned long long) * 256 * kGroupsMax, st));
@@ -961,8 +958,8 @@ int rmu_index_search(rmu_index* idx, const float* queries, int nq, int k, int64_
                 sp.epoch = ++idx->epoch;
             }
             sp.groups = keep / kPubRank;                      // 16 * groups >= keep rows score >= the exchanged threshold
-            if (grid < 2 * sp.groups) sp.groups = 0;          // small grids: lists are cut only by their own floors
-            rc = scan_dispatch(geo, idx->tmap, tq, sp, grid, st);
+            int grid = 0;
+            rc = scan_launch(idx, geo, qbase, nql, ntiles, sp, st, &grid);
             if (rc != RMU_OK) return rc;
             ++scan_launches;
             SelectParams fp{};
@@ -994,18 +991,10 @@ int rmu_index_search(rmu_index* idx, const float* queries, int nq, int k, int64_
             for (int j0 = 0; j0 < p2max;) {
                 const ScanGeom geo = scan_geometry(D, p2max - j0);
                 const int nql = std::min(p2max - j0, geo.nq);
-                const int grid = geo.pair ? 2 * std::min(idx->sms / 2, (ntiles + 1) / 2) : std::min(idx->sms, ntiles);
-                CUtensorMap tq;
-                rc = make_tmap_2d(&tq, d_qbuf + static_cast<size_t>(j0) * D, static_cast<uint64_t>(nql), static_cast<uint64_t>(D),
-                                  static_cast<uint64_t>(D) * sizeof(float), 32, static_cast<uint32_t>(geo.nq / (geo.pair ? 2 : 1)), 4);
-                if (rc != RMU_OK) return rc;
-                ScanParams sp{};
-                sp.nq = nql; sp.dim = D; sp.n = N; sp.ntiles = ntiles; sp.nstages = geo.nstages; sp.metric = idx->metric;
-                sp.rscale = idx->rscale; sp.rbias = idx->rbias; sp.stats_bits = idx->max_norm_bits;
-                sp.lists = d_scan; sp.counts = d_cnt; sp.floors = d_floor; sp.gmax = idx->gmax; sp.epoch = idx->epoch; sp.groups = 0;
+                ScanParams sp{};                              // pool mode: no lists, no exchange
                 sp.fixed_tau = d_taub + j0; sp.pool = d_pool + static_cast<size_t>(j0) * kPass2PoolCap; sp.pool_cnt = d_pcnt + j0;
                 sp.pool_cap = kPass2PoolCap; sp.nq_dev = d_nsel; sp.q_off = j0;
-                rc = scan_dispatch(geo, idx->tmap, tq, sp, grid, st);
+                rc = scan_launch(idx, geo, d_qbuf + static_cast<size_t>(j0) * D, nql, ntiles, sp, st);
                 if (rc != RMU_OK) return rc;
                 j0 += nql;
             }
@@ -1086,20 +1075,13 @@ int rmu_debug_scan_tile(rmu_index* idx, const float* queries, int nq, float* out
     if (rc != RMU_OK) return rc;
     rc = ensure_corpus_tmap(idx);
     if (rc != RMU_OK) return rc;
-    ScanGeom geo = scan_geometry(idx->dim, 64);
-    CUtensorMap tq;
-    rc = make_tmap_2d(&tq, queries, static_cast<uint64_t>(nq), static_cast<uint64_t>(idx->dim),
-                      static_cast<uint64_t>(idx->dim) * sizeof(float), 32, static_cast<uint32_t>(geo.nq / (geo.pair ? 2 : 1)), 4);
-    if (rc != RMU_OK) return rc;
     ScanParams sp{};
-    sp.nq = nq; sp.dim = idx->dim; sp.n = idx->n; sp.ntiles = 2; sp.nstages = geo.nstages; sp.metric = RMU_METRIC_IP;
-    sp.stats_bits = idx->max_norm_bits;
     sp.lists = static_cast<unsigned long long*>(idx->ws);
     sp.counts = reinterpret_cast<int*>(static_cast<uint8_t*>(idx->ws) + lists);
     sp.floors = reinterpret_cast<float*>(sp.counts + 128);
-    sp.gmax = idx->gmax; sp.epoch = ++idx->epoch; sp.groups = 0;
+    sp.epoch = ++idx->epoch;
     sp.dbg = out;
-    rc = scan_dispatch(geo, idx->tmap, tq, sp, 2, st);
+    rc = scan_launch(idx, scan_geometry(idx->dim, 64), queries, nq, 2, sp, st);   // two tiles: grid 2
     RMU_CUDA(cudaEventRecord(idx->ws_done, st));
     return rc;
 }

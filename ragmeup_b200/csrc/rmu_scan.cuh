@@ -44,6 +44,7 @@ constexpr int kGroupsMax = 16;                   // gmax row length; KSEL <= 16 
 constexpr int kScanStateBytes = 2048;            // mbarriers + per-query state behind the ring
 constexpr int kScanQOpMax = 96 * 1024;           // shared memory the resident half of the query operand may take
 constexpr int kScanMaxStages = 16;
+constexpr int kScanKD = 2;                       // TMA boxes (K blocks) per pipeline stage
 constexpr int kScanMaxQ = 128;                   // queries per launch (MMA N)
 
 struct ScanParams {
@@ -51,7 +52,7 @@ struct ScanParams {
     int dim;
     long long n;               // rows in the index
     int ntiles;                // ceil(n / 128)
-    int nstages;               // ring depth, in stages of KD boxes
+    int nstages;               // ring depth, in stages of kScanKD boxes
     int metric;
     const float* rscale;       // [n] 1/||x|| (cosine), used unless the corpus is unit-norm
     const float* rbias;        // [n] -0.5 ||x||^2 (L2), used unless the corpus is unit-norm
@@ -71,7 +72,6 @@ struct ScanParams {
     int pool_cap;
     const int* nq_dev;         // nullable: live queries of the pass (device count of flagged queries)
     int q_off;                 // this launch serves slots q_off .. q_off + nq - 1 of them
-    int ablate;                // profiling only: bit0 skip the MMAs, bit1 skip the epilogue work
 };
 
 // sort one candidate list (n <= 32 * E entries) descending, keep its best kListKeep, publish its kPubRank-th key
@@ -116,12 +116,12 @@ __device__ __forceinline__ void mma_tf32_ss_pair(uint32_t d_tmem, uint64_t a_des
 //   acc_empty[b] (leader's): one arrival per epilogue warp of either CTA;
 //   qbar (leader's): the resident query halves of both CTAs, same scheme as full[].
 // PAIR = false: one CTA, cta_group::1, the whole query block resident.
-template <int NQ, int KD, bool PAIR>
+template <int NQ, bool PAIR>
 __global__ void __launch_bounds__(64 + 32 * scan_epi_warps(NQ), 1)
 scan_rows_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_q, const ScanParams p) {
     constexpr int NCTA = PAIR ? 2 : 1;
     constexpr int NQH = NQ / NCTA;                       // query rows resident in THIS CTA
-    constexpr int STAGE_BYTES = KD * kBoxBytes;
+    constexpr int STAGE_BYTES = kScanKD * kBoxBytes;
     constexpr int QBLK_BYTES = NQH * 128;                // one K block of this CTA's part of the query operand
     constexpr int CW = NQ < 32 ? NQ : 32;                // accumulator columns per TMEM load
     constexpr int EPW = scan_epi_warps(NQ);              // epilogue warps: with 8, each TMEM lane quadrant has two, half the queries each
@@ -135,7 +135,7 @@ scan_rows_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_consta
     // 1024-byte alignment by OFFSET (a pointer round-trip through an integer loses the shared address space)
     uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
     const int KB = (p.dim + 31) / 32;                    // 128-byte K blocks
-    const int NST = (KB + KD - 1) / KD;                  // pipeline stages per tile
+    const int NST = (KB + kScanKD - 1) / kScanKD;        // pipeline stages per tile
     uint8_t* qop = smem;
     uint8_t* ring = smem + KB * QBLK_BYTES;
     uint8_t* state = ring + p.nstages * STAGE_BYTES;
@@ -197,11 +197,11 @@ scan_rows_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_consta
                     mbar_wait(&empty[slot], phase ^ 1);
                     if (rank == 0) mbar_arrive_expect_tx(&full[slot], NCTA * STAGE_BYTES);
 #pragma unroll
-                    for (int kk = 0; kk < KD; ++kk) {
+                    for (int kk = 0; kk < kScanKD; ++kk) {
                         // K blocks past the row end are out of bounds: they arrive as zeros and still count their bytes
                         uint8_t* dst = ring + slot * STAGE_BYTES + kk * kBoxBytes;
-                        if (PAIR) tma_load_2d_pair(dst, &tmap_x, (s * KD + kk) * 32, t * kTileRows, &full[slot], kEvictFirst);
-                        else tma_load_2d(dst, &tmap_x, (s * KD + kk) * 32, t * kTileRows, &full[slot], kEvictFirst);
+                        if (PAIR) tma_load_2d_pair(dst, &tmap_x, (s * kScanKD + kk) * 32, t * kTileRows, &full[slot], kEvictFirst);
+                        else tma_load_2d(dst, &tmap_x, (s * kScanKD + kk) * 32, t * kTileRows, &full[slot], kEvictFirst);
                     }
                     if (++slot == p.nstages) { slot = 0; phase ^= 1; }
                 }
@@ -225,9 +225,9 @@ scan_rows_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_consta
                     mbar_wait(&full[slot], phase);
                     tc_fence_after();
 #pragma unroll
-                    for (int kk = 0; kk < KD; ++kk) {
-                        const int kb = s * KD + kk;
-                        if (kb < KB && !(p.ablate & 1)) {
+                    for (int kk = 0; kk < kScanKD; ++kk) {
+                        const int kb = s * kScanKD + kk;
+                        if (kb < KB) {
                             const uint64_t adesc = umma_desc_sw128_kmajor(smem_u32(ring + slot * STAGE_BYTES + kk * kBoxBytes));
                             const uint64_t bdesc = umma_desc_sw128_kmajor(smem_u32(qop + kb * QBLK_BYTES));
 #pragma unroll
@@ -293,7 +293,6 @@ scan_rows_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_consta
                         else mbar_arrive(&acc_empty[buf]);
                     }
                 }
-                if (p.ablate & 2) continue;
                 if (p.dbg != nullptr && i == 0 && NCTA * unit + rank < 2) {     // tiles 0 and 1 = the first 256 rows
 #pragma unroll
                     for (int j = 0; j < CW; ++j) p.dbg[(c * CW + j) * 2 * kTileRows + (NCTA * unit + rank) * kTileRows + er] = __uint_as_float(r[j]);
@@ -330,7 +329,7 @@ scan_rows_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_consta
                     }
                 }
             }
-            if ((p.ablate & 2) || pool_mode) continue;
+            if (pool_mode) continue;
             // ---- tile boundary: sort + cut the lists that grew past kListTrig (every sort publishes the list's 16th key, so
             // the thresholds of all CTAs rise together: ~5 sorts per list over a 10M-row scan, most of them in the first tiles)
             const bool any = bar_red_or_named(1, ETH, mine);

@@ -58,29 +58,47 @@ def test_logits_match_hf_golden(cuda, golden_dir, preset, seed, scale):
     assert np.abs(enc.classify_host(ids, typ, cu) - lg).max() < 1e-6
 
 
-def test_ragged_batch_vs_oracle_long_sequences(cuda):
-    """S up to 512 (truncation limit), 150-token rerank-shaped pairs, single-token edge"""
+def _ragged_batch_vs_oracle(preset, head, lens, alone):
+    """one ragged batch through the encoder vs the oracle (logits with the classifier head, else normalised mean
+    embeddings), then the sequences `alone` re-run one at a time"""
     from ragmeup_b200.encoder import BertEncoder
-    preset = "ms-marco-MiniLM-L-6-v2"
     cfg = BertConfig(**asdict(PRESETS[preset][0]))
     ocfg = bert_ref.BertCfg(**asdict(cfg))
-    w = synthetic_bert_weights(cfg, seed=5, with_head=True, scale=4.0)
-    enc = BertEncoder(cfg, w, with_head=True)
+    w = synthetic_bert_weights(cfg, seed=5, with_head=head, scale=4.0)
+    enc = BertEncoder(cfg, w, with_head=head)
     rng = np.random.default_rng(9)
-    lens = [512, 147, 147, 2, 300, 31]
     ids = np.concatenate([np.r_[101, rng.integers(104, cfg.vocab_size, n - 2), 102] for n in lens]).astype(np.int32)
     typ = np.concatenate([np.r_[np.zeros(n // 3, np.int32), np.ones(n - n // 3, np.int32)] for n in lens])
     cu = np.r_[0, np.cumsum(lens)].astype(np.int32)
-    lg = enc.classify_tokens(ids, typ, cu, max(lens)).cpu()
+
+    def run(i, t, c, mx):
+        return (enc.classify_tokens(i, t, c, mx) if head else enc.embed_tokens(i, t, c, mx, "mean", True)).cpu()
+
+    out = run(ids, typ, cu, max(lens))
     S = max(lens)
     I = np.zeros((len(lens), S), np.int64); M = np.zeros_like(I); T = np.zeros_like(I)
     for b, n in enumerate(lens):
         I[b, :n] = ids[cu[b]:cu[b + 1]]; T[b, :n] = typ[cu[b]:cu[b + 1]]; M[b, :n] = 1
     with torch.no_grad():
         h = bert_ref.bert_encoder_forward(w, ocfg, torch.from_numpy(I), torch.from_numpy(M), torch.from_numpy(T))
-        ref = bert_ref.classifier_head(w, h)
-    assert float((lg - ref).abs().max()) < TOL
-    # batch-composition invariance: each sequence alone gives the same logit
-    for b in (1, 3):
-        one = enc.classify_tokens(ids[cu[b]:cu[b + 1]], typ[cu[b]:cu[b + 1]], np.array([0, lens[b]], np.int32), lens[b]).cpu()
-        assert float((one[0] - lg[b]).abs().max()) < 1e-5
+        ref = bert_ref.classifier_head(w, h) if head else bert_ref.l2_normalize(bert_ref.pool(h, torch.from_numpy(M), "mean"))
+    assert float((out - ref).abs().max()) < TOL
+    # batch-composition invariance: each sequence alone gives the same result
+    for b in alone:
+        one = run(ids[cu[b]:cu[b + 1]], typ[cu[b]:cu[b + 1]], np.array([0, lens[b]], np.int32), lens[b])
+        assert float((one[0] - out[b]).abs().max()) < 1e-5
+
+
+def test_ragged_batch_vs_oracle_long_sequences(cuda):
+    """S up to 512 (truncation limit), 150-token rerank-shaped pairs, single-token edge"""
+    _ragged_batch_vs_oracle("ms-marco-MiniLM-L-6-v2", True, [512, 147, 147, 2, 300, 31], (1, 3))
+
+
+# The longest sequence picks the attention kernel: MiniLM (d_h = 32) takes the per-head tcgen05 kernel at 161-224
+# keys, bge-base (d_h = 64, embeddings) the mma.sync kernel past 192 keys.
+@pytest.mark.parametrize("preset,head,lens,alone", [
+    ("ms-marco-MiniLM-L-6-v2", True, [200, 147, 31, 2], (1, 3)),
+    ("bge-base-en-v1.5", False, [300, 64, 5], (1, 2)),
+], ids=["minilm-200-keys", "bge-base-300-keys"])
+def test_ragged_batch_vs_oracle_attention_kernels(cuda, preset, head, lens, alone):
+    _ragged_batch_vs_oracle(preset, head, lens, alone)

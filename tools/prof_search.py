@@ -3,7 +3,7 @@ import os, sys, time
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ragmeup_b200.index import FlatIndex, MODE_AUTO, MODE_TENSOR_NOFALLBACK
-MODE = MODE_TENSOR_NOFALLBACK if os.environ.get('RMU_SEARCH_NOFALLBACK') == '1' or os.environ.get('RMU_SCAN_ABLATE') else MODE_AUTO
+MODE = MODE_TENSOR_NOFALLBACK if os.environ.get('RMU_SEARCH_NOFALLBACK') == '1' else MODE_AUTO
 N = int(os.environ.get("PROF_N", 10_000_000)); Q = int(os.environ.get("PROF_Q", 128)); K = int(os.environ.get("PROF_K", 10)); D = int(os.environ.get("PROF_D", 384))
 IT = int(os.environ.get("PROF_ITERS", 3)); metric = os.environ.get("PROF_METRIC", "ip")
 dev = torch.device("cuda")
